@@ -44,8 +44,7 @@ X1M_ITEMS, X1M_USERS, X1M_DEG = 1000000, 5000000, 50.0
 GOLD = os.path.join(ROOT, "tests", "golden", "askubuntu_sample.npz")
 N_BENCH_BATCHES = 8   # distinct user batches cycled through by the timed steps (per GPU)
 CPU_BATCH_CAP = 1000  # users per step of the CPU baseline sample (dense fp32 [B, I] tensors)
-MIN_TIMED_S = 0.5     # the K-step timed block is repeated until this much device time has accumulated (median block reported)
-MAX_REPEATS = 200
+DUMP_ROWS = 4096      # --dump-outputs: item rows sampled from each [I, 600] matrix (2 x 9.8 MB; all of them are 2 x 48 MB at ML-20M)
 H0, H1, H2, H3 = 100, 150, 250, 300   # config.ini h0..h3_size
 LR, LAM = 1e-4, 1.0                    # config.ini LEARNING_RATE, GANLAMBDA
 
@@ -62,7 +61,12 @@ def parse():
     ap.add_argument("--cpu-steps", type=int, default=6, help="steps of the bounded CPU-baseline sample")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-graphs", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (losses, updated parameters)")
+    args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.config == "x1m"):
+        ap.error("--dump-outputs writes the GAN step of --impl b200; --impl reference and --config x1m are not covered")
+    return args
 
 
 def measured_peaks(key="hbm_gbs"):
@@ -244,6 +248,31 @@ def eval_throughput(engine, tabs, n_users=2000):
                      "median of 3 calls")
 
 
+def step_outputs(engine, batch, world):
+    """What a caller of the timed GAN step holds after its last step: the losses and the updated generator and discriminator
+    parameters in the reference's order, as host arrays. Of the two [I, 600] item matrices (W_q0 rows, W_p1 columns) the same
+    DUMP_ROWS items, drawn with a fixed seed, are kept. Under data parallelism a collective: every rank calls it."""
+    import numpy as np
+    import torch
+    engine.gather_master()
+    out = {"loss_" + k: np.float64(v) for k, v in engine.last_losses(batch, reduce=world > 1).items()}
+    items = np.sort(np.random.RandomState(0).choice(engine.I, min(DUMP_ROWS, engine.I), replace=False))
+    sel = torch.from_numpy(items).to(engine.device)
+    for name, p in zip(("W_q0", "W_q1", "W_p0", "W_p1", "b_q0", "b_q1", "b_p0", "b_p1"), engine.vae.params):
+        p = p[sel] if name == "W_q0" else p[:, sel] if name == "W_p1" else p
+        out["gen_" + name] = p.detach().float().cpu().numpy()
+    for name, p in zip(("w1", "b1", "w2", "b2", "w3", "b3", "w4", "b4"), engine.disc.d_params):
+        out["disc_" + name] = p.detach().float().cpu().numpy()
+    return out
+
+
+def save_outputs(out_dir, arrays):
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def cpu_baseline(tabs, n_steps, n_items):
     """The reference's CPU data flow (oracle/cpu_step.py) on a bounded sample of the same workload."""
     import torch
@@ -369,25 +398,19 @@ def run_x1m(args, rank, world, local_rank):
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    block_ms = []
-    launches = 0
-    while True:
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        barrier()
-        k0 = engine.kernels_launched
-        e0.record()
-        for i in range(args.steps):
-            step(i)
-        e1.record()
-        barrier()
-        t = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device="cuda")
-        if world > 1:
-            dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        block_ms.append(float(t.item()))
-        launches = engine.kernels_launched - k0
-        if sum(block_ms) >= MIN_TIMED_S * 1e3 or len(block_ms) >= MAX_REPEATS:
-            break
-    ms = sorted(block_ms)[len(block_ms) // 2]
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    barrier()
+    k0 = engine.kernels_launched
+    e0.record()
+    for i in range(args.steps):
+        step(i)
+    e1.record()
+    barrier()
+    t = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device="cuda")
+    if world > 1:
+        dist.all_reduce(t, op=dist.ReduceOp.MAX)
+    ms = float(t.item())
+    launches = engine.kernels_launched - k0
     # end to end: the batch's index arrays come from pinned host memory, the loss scalars go back, every step
     host_scal = torch.zeros(2, ops.NSCAL, dtype=torch.float32).pin_memory()
     barrier()
@@ -464,8 +487,7 @@ def run_x1m(args, rank, world, local_rank):
                                   frac=roof["G"]["frac"], traffic=None),
                     eval=dict(users_per_sec=1000 / t_eval, users=1000, ms=t_eval * 1e3, ndcg_at_100_random_init=float(np.mean(m["ndcg@100"])),
                               what="fold-in forward over the shards + local exact top-100 per shard + all-gather/merge of 100 (score, id) pairs per rank"),
-                    losses_last_step={k: float(v) for k, v in L.items()},
-                    timing=dict(repeats=len(block_ms), block_ms_min=min(block_ms), block_ms_median=ms, block_ms_max=max(block_ms)))
+                    losses_last_step={k: float(v) for k, v in L.items()}, timing=dict(timed_steps=args.steps, block_ms=ms))
         if world > 1:
             line["comm"] = dict(world_size=dist.get_world_size(), backend=dist.get_backend())
         print(json.dumps(line), flush=True)
@@ -542,28 +564,22 @@ def main():
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    # The timed region is EXACTLY args.steps steps between two barriers; it is repeated (each repeat timed on its own, same
-    # bracketing) until at least MIN_TIMED_S of device time has accumulated, and the MEDIAN repeat is reported: one 20-step block is
-    # ~10 ms, too short for the clock sampler and for run-to-run noise to show.
-    block_ms = []
-    launches = 0
-    while True:
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        barrier()
-        k0 = engine.kernels_launched
-        e0.record()
-        for i in range(args.steps):
-            step(i)
-        e1.record()
-        barrier()
-        t = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device="cuda")
-        if world > 1:
-            dist.all_reduce(t, op=dist.ReduceOp.MAX)   # every rank sees the same number, so every rank stops after the same repeat
-        block_ms.append(float(t.item()))
-        launches = engine.kernels_launched - k0
-        if sum(block_ms) >= MIN_TIMED_S * 1e3 or len(block_ms) >= MAX_REPEATS:
-            break
-    ms = sorted(block_ms)[len(block_ms) // 2]
+    # The timed region is exactly args.steps steps between two barriers, so the state the timed path leaves behind (and
+    # --dump-outputs writes) depends on the arguments alone.
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    barrier()
+    k0 = engine.kernels_launched
+    e0.record()
+    for i in range(args.steps):
+        step(i)
+    e1.record()
+    barrier()
+    t = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device="cuda")
+    if world > 1:
+        dist.all_reduce(t, op=dist.ReduceOp.MAX)
+    ms = float(t.item())
+    launches = engine.kernels_launched - k0
+    outputs = step_outputs(engine, BATCH, world) if args.dump_outputs else None   # before the steps below move the weights on
 
     # ---- end-to-end: the step's inputs come from pinned host memory, the losses go back to the host, every step ----
     # Software-pipelined like a real input pipeline: while step i computes, the inputs of step i+1 travel host->device on a
@@ -609,13 +625,7 @@ def main():
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return float(t.item()), h2d
 
-    e2e_ms = []
-    while True:
-        t, h2d = e2e_block()
-        e2e_ms.append(t)
-        if sum(e2e_ms) >= MIN_TIMED_S * 1e3 or len(e2e_ms) >= MAX_REPEATS:
-            break
-    ms_e2e = sorted(e2e_ms)[len(e2e_ms) // 2]
+    ms_e2e, h2d = e2e_block()
     clocks = sampler.stop() if rank == 0 else None
 
     # ---- per-phase split and the dominant kernel (fused Adam over the [I,600] decoder weight), CUDA events, same stream ----
@@ -736,10 +746,7 @@ def main():
                     gpu_launches=launches, clocks=clocks, roofline=roof,
                     phases_ms=dict(A=t_a, D=t_d, G=t_g, epoch_weighted_users_per_sec=BATCH * world / ((t_a + 10 * t_d + 10 * t_g) * 1e-3)),
                     pairs_per_step=dict(real=int(np.mean([b["Pr"] for b in data.batches])), generated_slots=int(np.mean([b["K"] for b in data.batches]))),
-                    graphs=not args.no_graphs,
-                    timing=dict(repeats=len(block_ms), block_ms_min=min(block_ms), block_ms_median=ms, block_ms_max=max(block_ms),
-                                e2e_repeats=len(e2e_ms), rule="the %d-step block is repeated until >= %.1f s of device time; median block reported"
-                                                              % (args.steps, MIN_TIMED_S)))
+                    graphs=not args.no_graphs, timing=dict(timed_steps=args.steps, block_ms=ms, e2e_block_ms=ms_e2e))
         if world > 1:
             line["dp_check"] = dp_res
             line["comm"] = dict(world_size=dist.get_world_size(), backend=dist.get_backend(), nccl_version=".".join(str(x) for x in torch.cuda.nccl.version()))
@@ -763,6 +770,8 @@ def main():
                 line["eval"] = dict(error=repr(e)[:200])
         if world == 1 and not args.no_cpu_baseline:
             line["cpu_baseline"] = cpu_baseline(tabs, args.cpu_steps, I)
+        if outputs is not None:
+            save_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
     if world > 1:
         # NCCL collectives live inside captured CUDA graphs; tearing the process group down under them can block, and

@@ -307,6 +307,17 @@ int ltg_disc_head(const void* Y3_bf16, int ld, int P, int h3, const float* w4, c
 int ltg_topk_metrics(const void* scores, int is_bf16, int64_t ld, int n_rows, int n_items,
                      const int32_t* seen_ptr, const int32_t* seen_items, const int32_t* held_ptr, const int32_t* held_items,
                      int k, const int32_t* rk_host, int n_rk, int32_t* topk_idx, double* dcg, int32_t* hits, void* stream);
+/* Recommendation lists. Per row u of fp32 logits (pitch ld; columns n_items..ld are never read), an item is ELIGIBLE when it is not in
+ * seen_items[seen_ptr[u] .. seen_ptr[u+1]) and its bit of allow_bits ((n_items+31)/32 words, bit i%32 of word i/32) is set. Excluded
+ * items are never listed. out_idx [n, k]: the min(k, #eligible) eligible items with the highest logits ordered by (logit desc, item id
+ * asc), the tie rule of ltg_topk_metrics; remaining slots -1. out_logit [n, k]: the listed logits, bit-equal to the input, -inf for
+ * padding. out_lse [n]: log sum_i exp(logit_i) over ALL n_items columns whatever the filters exclude (max-shifted, fp32, expf), so
+ * out_prob [n, k] (may be NULL) = exp(logit - lse) is the generator's softmax probability (MultiVAE.py:143), 0 for padding.
+ * 1 <= k <= 128. Rows of at most 49,152 items with 16-byte aligned rows are staged in shared memory; larger catalogs stream.        */
+int ltg_topk_recommend(const float* scores, int64_t ld, int n_rows, int n_items,
+                       const int32_t* seen_ptr, const int32_t* seen_items,   /* may both be NULL: nothing excluded */
+                       const uint32_t* allow_bits,                           /* may be NULL: every item allowed   */
+                       int k, int32_t* out_idx, float* out_logit, float* out_prob, float* out_lse, void* stream);
 
 /* ---- a1 / f3: dataset ingestion on the host cores (data_processing.py:6-37: pandas.read_csv + scipy csr_matrix) -----------
  * HOST entry points (no kernels, no stream): every pointer below is a host pointer.

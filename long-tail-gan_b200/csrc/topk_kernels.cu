@@ -460,3 +460,301 @@ extern "C" int ltg_topk_metrics(const void* scores, int is_bf16, int64_t ld, int
   LTG_CHECK_LAUNCH();
   return LTG_OK;
 }
+
+
+// ---------------------------------------------------------------------------------------------------------------------------------
+// Recommendation lists (ltg_topk_recommend): per row, the top k ELIGIBLE items of fp32 logits with their logits and softmax
+// probabilities. An item is eligible when it is not in the row's seen list and its bit of allow_bits is set. The metrics kernels above
+// turn seen items into -inf keys, which the selection can still pick; here an excluded item is never counted by the selection at all.
+// The probability is the softmax over the WHOLE catalog (MultiVAE.py:143, item_prob_dist): the row's log-sum-exp is taken over every
+// column before anything is excluded, so a filter chooses which items are listed and never renormalises their probabilities.
+// ---------------------------------------------------------------------------------------------------------------------------------
+namespace {
+
+// Excluded items of a staged row carry this key: it is the key of the negative NaN with every bit set, so no logit maps to it and it is
+// below every real key (a per-thread maximum over a thread's items is then a maximum over its eligible items, or this key if it has none).
+constexpr uint32_t KEY_EXCLUDED = 0u;
+
+__device__ __forceinline__ float ord2f(uint32_t key) { return __uint_as_float((key & 0x80000000u) ? (key & 0x7FFFFFFFu) : ~key); }
+
+// (m, s) = (max, sum exp(x - max)) of two partial sets -> the pair of their union
+__device__ __forceinline__ void lse_merge(float& m, float& s, float m2, float s2) {
+  const float M = fmaxf(m, m2);
+  if (M == -INFINITY) return;
+  s = (m == -INFINITY ? 0.f : s * expf(m - M)) + (m2 == -INFINITY ? 0.f : s2 * expf(m2 - M));
+  m = M;
+}
+
+// s_win (key << 32 | ~index, unused entries 0) -> sorted by (logit desc, index asc); the first kk entries are the list, the rest of the k
+// slots are padding (-1, -inf, 0)
+__device__ __forceinline__ void sort_and_write(unsigned long long* s_win, int u, int k, int kk, float lse, int32_t* out_idx, float* out_logit,
+                                               float* out_prob, float* out_lse) {
+  const int tid = threadIdx.x;
+  for (int size = 2; size <= TK_MAXK; size <<= 1) {
+    for (int stride = size >> 1; stride > 0; stride >>= 1) {
+      if (tid < TK_MAXK) {
+        const int j = tid ^ stride;
+        if (j > tid) {
+          const unsigned long long a = s_win[tid], b = s_win[j];
+          const bool desc = (tid & size) == 0;
+          if ((a < b) == desc) { s_win[tid] = b; s_win[j] = a; }
+        }
+      }
+      __syncthreads();
+    }
+  }
+  if (tid < k) {
+    const size_t o = (size_t)u * k + tid;
+    if (tid < kk) {
+      const unsigned long long w = s_win[tid];
+      const float x = ord2f((uint32_t)(w >> 32));   // f2ord is a bijection: the input's bits
+      out_idx[o] = (int)~(uint32_t)(w & 0xFFFFFFFFull);
+      out_logit[o] = x;
+      if (out_prob != nullptr) out_prob[o] = expf(x - lse);
+    } else {
+      out_idx[o] = -1;
+      out_logit[o] = -INFINITY;
+      if (out_prob != nullptr) out_prob[o] = 0.f;
+    }
+  }
+  if (tid == 0) out_lse[u] = lse;
+}
+
+// Staged path (n_items <= TS_MAX_ITEMS, 16-byte aligned rows): the row is read once into shared memory as keys; max and sum-exp are
+// taken over the raw values, then excluded items are overwritten with KEY_EXCLUDED and the selection skips that key through the
+// predicate of radix_select11. The candidate pre-filter of topk_staged_kernel stays exact because its per-thread maxima are maxima over
+// eligible items (a maximum over excluded ones could raise the bound above the kk-th eligible logit and drop winners).
+__global__ void __launch_bounds__(TS_THREADS)
+topk_rec_staged_kernel(const float* __restrict__ scores, int64_t ld, int n_items, const int32_t* __restrict__ seen_ptr,
+                       const int32_t* __restrict__ seen_items, const uint32_t* __restrict__ allow_bits, int k, int32_t* __restrict__ out_idx,
+                       float* __restrict__ out_logit, float* __restrict__ out_prob, float* __restrict__ out_lse) {
+  extern __shared__ __align__(16) uint32_t s_keys[];   // [n_items rounded up to 8]
+  __shared__ __align__(16) uint32_t s_hist[TS_BINS];
+  __shared__ uint32_t s_warp[TS_THREADS / 32];
+  __shared__ float s_wsum[TS_THREADS / 32];
+  __shared__ uint32_t s_sel[3];
+  __shared__ uint32_t s_lmax[TS_THREADS];
+  __shared__ unsigned long long s_cand[TS_CAND];
+  __shared__ int s_ncand;
+  __shared__ unsigned long long s_win[TK_MAXK];
+  __shared__ int s_nwin;
+
+  const int u = blockIdx.x;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  if (tid < TK_MAXK) s_win[tid] = 0ull;
+  if (tid == 0) { s_nwin = 0; s_ncand = 0; }
+  // ---- the row, once, 16 bytes per load (as topk_staged_kernel), and its largest key
+  const float* row = scores + (size_t)u * ld;
+  const int n4 = n_items >> 2;
+  uint32_t kmax = 0u;
+  for (int v0 = 0; v0 < n4; v0 += TS_LD * TS_THREADS) {
+    uint4 x[TS_LD];
+#pragma unroll
+    for (int q = 0; q < TS_LD; ++q) {
+      const int v = v0 + q * TS_THREADS + tid;
+      if (v < n4) x[q] = ld_nc_v4(reinterpret_cast<const uint4*>(row) + v);
+    }
+#pragma unroll
+    for (int q = 0; q < TS_LD; ++q) {
+      const int v = v0 + q * TS_THREADS + tid;
+      if (v < n4) {
+        uint4 o;
+        o.x = f2ord(__uint_as_float(x[q].x)); o.y = f2ord(__uint_as_float(x[q].y)); o.z = f2ord(__uint_as_float(x[q].z));
+        o.w = f2ord(__uint_as_float(x[q].w));
+        kmax = max(kmax, max(max(o.x, o.y), max(o.z, o.w)));
+        *reinterpret_cast<uint4*>(s_keys + 4 * v) = o;
+      }
+    }
+  }
+  for (int i = (n4 << 2) + tid; i < n_items; i += TS_THREADS) {
+    const uint32_t key = f2ord(row[i]);
+    s_keys[i] = key;
+    kmax = max(kmax, key);
+  }
+  kmax = __reduce_max_sync(0xffffffffu, kmax);
+  if (lane == 0) s_warp[warp] = kmax;
+  __syncthreads();
+  kmax = 0u;
+#pragma unroll
+  for (int w = 0; w < TS_THREADS / 32; ++w) kmax = max(kmax, s_warp[w]);
+  const float mx = ord2f(kmax);
+  // ---- sum-exp over every column (fixed order: bit-reproducible), and the allow filter in the same pass
+  float se = 0.f;
+  for (int i = tid; i < n_items; i += TS_THREADS) {
+    se += expf(ord2f(s_keys[i]) - mx);
+    if (allow_bits != nullptr && !((allow_bits[i >> 5] >> (i & 31)) & 1u)) s_keys[i] = KEY_EXCLUDED;
+  }
+  se = warp_sum(se);
+  if (lane == 0) s_wsum[warp] = se;
+  __syncthreads();
+  float S = 0.f;
+#pragma unroll
+  for (int w = 0; w < TS_THREADS / 32; ++w) S += s_wsum[w];
+  const float lse = mx + logf(S);
+  if (seen_ptr != nullptr)
+    for (int j = seen_ptr[u] + tid; j < seen_ptr[u + 1]; j += TS_THREADS) s_keys[seen_items[j]] = KEY_EXCLUDED;
+  __syncthreads();
+  // ---- number of eligible items and the pre-filter's per-thread maxima, both over eligible items only
+  uint32_t lmax = 0u, cnt = 0u;
+  for (int i = tid; i < n_items; i += TS_THREADS) {
+    const uint32_t key = s_keys[i];
+    lmax = max(lmax, key);
+    cnt += key != KEY_EXCLUDED;
+  }
+  s_lmax[tid] = lmax;
+  cnt = __reduce_add_sync(0xffffffffu, cnt);
+  if (lane == 0) s_warp[warp] = cnt;
+  __syncthreads();
+  uint32_t n_elig = 0u;
+#pragma unroll
+  for (int w = 0; w < TS_THREADS / 32; ++w) n_elig += s_warp[w];
+  const int kk = min(k, (int)n_elig);
+  if (kk > 0) {   // (uniform over the CTA)
+    uint32_t c0 = 0, k0 = 0;
+    const uint32_t bound = radix_select11(TS_THREADS, (uint32_t)kk, [&](int i, uint32_t& v) { v = s_lmax[i]; return true; }, s_hist, s_warp,
+                                          s_sel, &c0, &k0);
+    for (int i = tid; i < n_items; i += TS_THREADS) {
+      const uint32_t key = s_keys[i];
+      if (key >= bound && key != KEY_EXCLUDED) {
+        const int slot = atomicAdd(&s_ncand, 1);
+        if (slot < TS_CAND) s_cand[slot] = ((unsigned long long)key << 32) | (unsigned long long)(~(uint32_t)i);
+      }
+    }
+    __syncthreads();
+    const bool use_cand = s_ncand <= TS_CAND;   // overflow (massive ties): select over the whole row, same result
+    const int n_el = use_cand ? s_ncand : n_items;
+    auto key_of = [&](int i) -> uint32_t { return use_cand ? (uint32_t)(s_cand[i] >> 32) : s_keys[i]; };
+    auto inv_of = [&](int i) -> uint32_t { return use_cand ? (uint32_t)(s_cand[i] & 0xFFFFFFFFull) : ~(uint32_t)i; };
+    uint32_t cnt_eq = 0, k_rem = 0;
+    const uint32_t T = radix_select11(n_el, (uint32_t)kk, [&](int i, uint32_t& v) { v = key_of(i); return v != KEY_EXCLUDED; }, s_hist, s_warp,
+                                      s_sel, &cnt_eq, &k_rem);
+    // ties at the threshold: keep the k_rem lowest indices among the cnt_eq eligible elements equal to T (T is never KEY_EXCLUDED)
+    uint32_t inv_thr = 0u;
+    if (cnt_eq != k_rem) {
+      uint32_t c2 = 0, k2 = 0;
+      inv_thr = radix_select11(n_el, k_rem, [&](int i, uint32_t& v) { v = inv_of(i); return key_of(i) == T; }, s_hist, s_warp, s_sel, &c2, &k2);
+    }
+    for (int i = tid; i < n_el; i += TS_THREADS) {
+      const uint32_t key = key_of(i), inv = inv_of(i);
+      if (key > T || (key == T && inv >= inv_thr)) {
+        const int slot = atomicAdd(&s_nwin, 1);
+        if (slot < TK_MAXK) s_win[slot] = ((unsigned long long)key << 32) | (unsigned long long)inv;
+      }
+    }
+  }
+  __syncthreads();
+  sort_and_write(s_win, u, k, kk, lse, out_idx, out_logit, out_prob, out_lse);
+}
+
+// Streaming path (larger catalogs, e.g. a 1 M-item catalog or one 125 k-item shard of it): one exclusion bitmap per row in shared memory
+// (the complement of allow_bits, then the seen items OR-ed in: n_items / 8 bytes, 125 KB at 1 M items), one online max / sum-exp pass
+// over the row, then the 8-bit radix select of topk_metrics_kernel over the eligible items only.
+__global__ void __launch_bounds__(TK_THREADS)
+topk_rec_stream_kernel(const float* __restrict__ scores, int64_t ld, int n_items, const int32_t* __restrict__ seen_ptr,
+                       const int32_t* __restrict__ seen_items, const uint32_t* __restrict__ allow_bits, int k, int32_t* __restrict__ out_idx,
+                       float* __restrict__ out_logit, float* __restrict__ out_prob, float* __restrict__ out_lse) {
+  extern __shared__ uint32_t s_excl[];   // [(n_items+31)/32]: bit set = excluded
+  __shared__ uint32_t s_hist[256];
+  __shared__ uint32_t s_sel[3];
+  __shared__ float2 s_ms[TK_THREADS / 32];
+  __shared__ uint32_t s_cnt[TK_THREADS / 32];
+  __shared__ unsigned long long s_win[TK_MAXK];
+  __shared__ int s_nwin;
+
+  const int u = blockIdx.x;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const float* row = scores + (size_t)u * ld;
+  const int words = (n_items + 31) >> 5;
+  for (int w = tid; w < words; w += TK_THREADS) s_excl[w] = allow_bits != nullptr ? ~allow_bits[w] : 0u;
+  if (tid < TK_MAXK) s_win[tid] = 0ull;
+  if (tid == 0) s_nwin = 0;
+  __syncthreads();
+  if (seen_ptr != nullptr)
+    for (int j = seen_ptr[u] + tid; j < seen_ptr[u + 1]; j += TK_THREADS) {
+      const int it = seen_items[j];
+      atomicOr(&s_excl[it >> 5], 1u << (it & 31));
+    }
+  __syncthreads();
+  auto eligible = [&](int i) -> bool { return !((s_excl[i >> 5] >> (i & 31)) & 1u); };
+  // ---- online max / sum-exp over every column, and the number of eligible items
+  float m = -INFINITY, s = 0.f;
+  uint32_t cnt = 0u;
+  for (int i = tid; i < n_items; i += TK_THREADS) {
+    const float x = row[i];
+    if (x > m) { s = s * expf(m - x) + 1.f; m = x; }
+    else if (m != -INFINITY) s += expf(x - m);
+    cnt += eligible(i);
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const float m2 = __shfl_down_sync(0xffffffffu, m, o), s2 = __shfl_down_sync(0xffffffffu, s, o);
+    lse_merge(m, s, m2, s2);
+  }
+  cnt = __reduce_add_sync(0xffffffffu, cnt);
+  if (lane == 0) { s_ms[warp] = make_float2(m, s); s_cnt[warp] = cnt; }
+  __syncthreads();
+  float M = s_ms[0].x, S = s_ms[0].y;
+  uint32_t n_elig = s_cnt[0];
+#pragma unroll
+  for (int w = 1; w < TK_THREADS / 32; ++w) { lse_merge(M, S, s_ms[w].x, s_ms[w].y); n_elig += s_cnt[w]; }
+  const float lse = M + logf(S);
+  const int kk = min(k, (int)n_elig);
+  if (kk > 0) {   // (uniform over the CTA)
+    uint32_t cnt_eq = 0, k_rem = 0;
+    const uint32_t T = radix_select_desc(n_items, (uint32_t)kk, [&](int i, uint32_t& v) { v = f2ord(row[i]); return eligible(i); }, s_hist,
+                                         s_sel, &cnt_eq, &k_rem);
+    uint32_t inv_thr = 0u;
+    if (cnt_eq != k_rem) {
+      uint32_t c2 = 0, k2 = 0;
+      inv_thr = radix_select_desc(n_items, k_rem, [&](int i, uint32_t& v) { v = ~(uint32_t)i; return eligible(i) && f2ord(row[i]) == T; },
+                                  s_hist, s_sel, &c2, &k2);
+    }
+    for (int i = tid; i < n_items; i += TK_THREADS) {
+      if (!eligible(i)) continue;
+      const uint32_t key = f2ord(row[i]);
+      if (key > T || (key == T && ~(uint32_t)i >= inv_thr)) {
+        const int slot = atomicAdd(&s_nwin, 1);
+        if (slot < TK_MAXK) s_win[slot] = ((unsigned long long)key << 32) | (unsigned long long)(~(uint32_t)i);
+      }
+    }
+  }
+  __syncthreads();
+  sort_and_write(s_win, u, k, kk, lse, out_idx, out_logit, out_prob, out_lse);
+}
+
+}  // namespace
+
+extern "C" int ltg_topk_recommend(const float* scores, int64_t ld, int n_rows, int n_items, const int32_t* seen_ptr, const int32_t* seen_items,
+                                  const uint32_t* allow_bits, int k, int32_t* out_idx, float* out_logit, float* out_prob, float* out_lse,
+                                  void* stream) {
+  LTG_REQUIRE(scores && out_idx && out_logit && out_lse);
+  LTG_REQUIRE(k >= 1 && k <= TK_MAXK && n_items >= 1 && ld >= n_items);
+  LTG_REQUIRE(seen_ptr == nullptr || seen_items != nullptr);
+  if (n_rows <= 0) return LTG_OK;
+  const bool aligned = (reinterpret_cast<uintptr_t>(scores) & 15) == 0 && ((ld * 4) & 15) == 0;
+  if (n_items <= TS_MAX_ITEMS && aligned) {
+    const size_t sm = (size_t)((n_items + 7) / 8 * 8) * 4;
+    static size_t opted_s = 16 * 1024;   // the kernel has ~28 KB of static shared memory
+    if (sm > opted_s) {
+      const cudaError_t e = cudaFuncSetAttribute(topk_rec_staged_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+      if (e != cudaSuccess) { ltg_set_last_error(cudaGetErrorString(e), __FILE__, __LINE__); return LTG_ERR_CUDA; }
+      opted_s = sm;
+    }
+    topk_rec_staged_kernel<<<n_rows, TS_THREADS, sm, (cudaStream_t)stream>>>(scores, ld, n_items, seen_ptr, seen_items, allow_bits, k, out_idx,
+                                                                             out_logit, out_prob, out_lse);
+    LTG_CHECK_LAUNCH();
+    return LTG_OK;
+  }
+  const size_t smem = (size_t)((n_items + 31) / 32) * 4;
+  LTG_REQUIRE(smem <= 200 * 1024);
+  static size_t opted = 40 * 1024;
+  if (smem > opted) {
+    const cudaError_t e = cudaFuncSetAttribute(topk_rec_stream_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) { ltg_set_last_error(cudaGetErrorString(e), __FILE__, __LINE__); return LTG_ERR_CUDA; }
+    opted = smem;
+  }
+  topk_rec_stream_kernel<<<n_rows, TK_THREADS, smem, (cudaStream_t)stream>>>(scores, ld, n_items, seen_ptr, seen_items, allow_bits, k, out_idx,
+                                                                             out_logit, out_prob, out_lse);
+  LTG_CHECK_LAUNCH();
+  return LTG_OK;
+}

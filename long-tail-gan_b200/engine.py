@@ -20,6 +20,31 @@ def _pad(n, q):
     return (n + q - 1) // q * q
 
 
+def allow_mask(allow, n_items):
+    """`allow` as an iterable of item ids or a boolean mask of length n_items -> boolean mask [n_items]."""
+    a = allow if isinstance(allow, np.ndarray) else np.asarray(list(allow))
+    if a.dtype == bool:
+        if a.shape != (n_items,):
+            raise ValueError("a boolean allow mask must have shape (%d,), got %s" % (n_items, a.shape))
+        return a
+    ids = a.astype(np.int64).reshape(-1)
+    if ids.size and (ids.min() < 0 or ids.max() >= n_items):
+        raise ValueError("allowed item ids must lie in [0, %d)" % n_items)
+    m = np.zeros(n_items, dtype=bool)
+    m[ids] = True
+    return m
+
+
+def allow_bits(allow, n_items, lo=0, hi=None):
+    """The allow bitmap of ltg_topk_recommend for items [lo, hi) of an n_items catalog (a catalog shard; default the whole catalog):
+    uint32 words, bit j % 32 of word j // 32 set when item lo + j is allowed. A shard packs from the global set, since its bounds need
+    not be multiples of 32."""
+    hi = n_items if hi is None else hi
+    m = allow_mask(allow, n_items)[lo:hi]
+    m = np.concatenate([m, np.zeros(-len(m) % 32, dtype=bool)])
+    return np.packbits(m, bitorder="little").view("<u4").astype(np.uint32)
+
+
 class TrainData(object):
     """Everything phase A/D/G need about the training users, resident on the device, plus per-batch index structures.
 
@@ -1095,22 +1120,36 @@ class GanEngine(object):
     # ------------------------------------------------------------------------------------------------------------
     # evaluation: train.py:333-348, test.py:138-173 + eval_functions.py
     # ------------------------------------------------------------------------------------------------------------
+    def _eval_batch(self, N, batch):
+        """Users per evaluation launch. Default: up to 4,096, bounded by 1 GiB of fp32 scores (the reference's batch_size_vad /
+        batch_size_test only bound its dense host arrays, train.py:333-337; every user is scored independently, dropout keyed by user id)."""
+        cap = max(1, min(4096, (1 << 30) // (4 * self.ld)))
+        if batch is None:
+            nbat = max(1, -(-N // cap))
+            return max(1, -(-N // nbat))          # equal batches (10,000 users -> 3 x 3,334, not 4,096 + 4,096 + 1,808)
+        return max(1, min(int(batch), cap))
+
+    def _eval_forward(self, ws, trp, tri, coef, b0, B, uid0, keep, max_nnz, words, scal):
+        """One batch of the inference forward (MultiVAE.forward_pass at is_training = 0, MultiVAE.py:175-186): rng-step advance, encoder
+        gather of fold-in rows [b0, b0 + B) -> middle -> fp32 decoder GEMM into ws.scores. `words` / `scal` are the step state it advances
+        and reads: the engine's own for evaluate, private copies for recommend. Returns the batch's row pointers."""
+        v = self.vae
+        ops.step_advance(words, scal, 0, self.lr)
+        ip = trp[b0: b0 + B + 1]
+        ops.enc_gather_fwd(ip, tri, None, B, self.I, uid0, v.W_q0_b, v.view("b_q0"), keep, self.seed, 0, words, ws.h1, coef, max_nnz,
+                           ws.enc_ws, ws.enc_cnt)
+        self._middle_unfused(B, uid0, 0.0, words, scal, ws=ws)
+        ops.gemm(ws.h2, v.WdT_b, B, self.I, H, bn=256, out_f32=ws.scores, bias=v.view("b_p1"))
+        return ip
+
     def evaluate(self, tr_indptr, tr_indices, te_indptr, te_indices, k=100, recall_ks=(20, 50), batch=None, uid_start=0, keep=None):
         """Scores every eval user from its fold-in interactions, masks them, ranks, and returns the per-user lists
         (ndcg@k, recall@rk...) over users with a non-empty held-out set, exactly like eval_functions.py."""
         dev = self.device
         N = len(tr_indptr) - 1
-        # default batch: up to 4,096 users, bounded by 1 GiB of fp32 scores (the reference's batch_size_vad / batch_size_test only bound
-        # its dense host arrays, train.py:333-337; every user is scored independently, dropout keyed by user id)
-        cap = max(1, min(4096, (1 << 30) // (4 * self.ld)))
-        if batch is None:
-            nbat = max(1, -(-N // cap))
-            batch = max(1, -(-N // nbat))          # equal batches (10,000 users -> 3 x 3,334, not 4,096 + 4,096 + 1,808)
-        else:
-            batch = max(1, min(int(batch), cap))
+        batch = self._eval_batch(N, batch)
         ws = self._eval_workspace(batch)
         keep = self.keep_vae if keep is None else keep
-        v = self.vae
         scores = ws.scores
         tr_ptr_h = np.ascontiguousarray(tr_indptr, dtype=np.int32)
         tr_idx_h = torch.from_numpy(np.ascontiguousarray(tr_indices if len(tr_indices) else np.zeros(1), dtype=np.int32))
@@ -1147,13 +1186,8 @@ class GanEngine(object):
 
         for b0 in range(0, N, batch):
             B = min(batch, N - b0)
-            ops.step_advance(self.words, self.scal, 0, self.lr)
-            ip = trp[b0: b0 + B + 1]
-            ops.enc_gather_fwd(ip, tri, None, B, self.I, uid_start + b0, v.W_q0_b, v.view("b_q0"), keep, self.seed, 0, self.words,
-                               ws.h1, coef, max_eval_nnz, ws.enc_ws, ws.enc_cnt)
-            self._middle_unfused(B, uid_start + b0, 0.0, self.words, self.scal, ws=ws)
             # fp32 logits: softmax is monotone per row, so ranking the logits equals ranking generator_out (SURVEY section 7)
-            ops.gemm(ws.h2, v.WdT_b, B, self.I, H, bn=256, out_f32=scores, bias=v.view("b_p1"))
+            ip = self._eval_forward(ws, trp, tri, coef, b0, B, uid_start + b0, keep, max_eval_nnz, self.words, self.scal)
             if b0 == 0:
                 upload_rest()
             ops.topk_metrics(scores, B, self.I, ip, tri, state["tep"][b0: b0 + B + 1], state["tei"], k, recall_ks, None, state["dcg"][b0:],
@@ -1163,6 +1197,41 @@ class GanEngine(object):
         dcg, hits = state["dcg"], state["hits"][:, :len(recall_ks)]
         torch.cuda.synchronize()
         return metrics_from_counts(dcg.cpu().numpy(), hits.cpu().numpy(), np.diff(np.asarray(te_indptr, dtype=np.int64)), k, recall_ks)
+
+    def recommend(self, tr_indptr, tr_indices, k=100, batch=None, uid_start=0, keep=1.0, exclude_seen=True, allow=None):
+        """Top-k recommendation lists for the users whose fold-in interactions are the CSR rows (tr_indptr, tr_indices). Users are scored
+        exactly as `evaluate` scores them (same batches, dropout keyed by uid_start + row); keep=1.0 (default) gives deterministic lists,
+        keep=None the engine's keep_vae (the reference's inference default). exclude_seen: never list a fold-in item. allow (optional): an
+        iterable of item ids or a boolean mask of length I; only those items are listed. Returns NumPy arrays: items int64 [N, k] ordered
+        by probability (ties: lower id first; -1 pads a row with fewer than k eligible items), probs float32 [N, k] (the generator's
+        softmax over the whole catalog, MultiVAE.py:143: a filter does not renormalise them; 0 for padding), lse float32 [N] (the row's
+        log-sum-exp of the logits). The engine's rng step and scalars are left as they were: the forward advances private copies."""
+        dev = self.device
+        N = len(tr_indptr) - 1
+        batch = self._eval_batch(N, batch)
+        ws = self._eval_workspace(batch)
+        keep = self.keep_vae if keep is None else float(keep)
+        tr_ptr_h = np.ascontiguousarray(tr_indptr, dtype=np.int32)
+        tr_idx_h = np.ascontiguousarray(tr_indices if len(tr_indices) else np.zeros(1), dtype=np.int32)
+        if len(tr_indices) and (tr_idx_h.min() < 0 or tr_idx_h.max() >= self.I):
+            raise ValueError("fold-in item ids must lie in [0, %d)" % self.I)
+        trp = torch.as_tensor(tr_ptr_h).to(dev)
+        tri = torch.as_tensor(tr_idx_h).to(dev)
+        coef = torch.empty(tri.numel(), dtype=torch.float32, device=dev)
+        max_nnz = int(np.diff(tr_ptr_h.astype(np.int64)).max()) if N > 0 else 0
+        bits = None if allow is None else torch.from_numpy(allow_bits(allow, self.I).view(np.int32)).to(dev)
+        words, scal = self.words.clone(), self.scal.clone()
+        items = torch.empty(N, k, dtype=torch.int32, device=dev)
+        logits = torch.empty(N, k, dtype=torch.float32, device=dev)
+        probs = torch.empty(N, k, dtype=torch.float32, device=dev)
+        lse = torch.empty(N, dtype=torch.float32, device=dev)
+        for b0 in range(0, N, batch):
+            B = min(batch, N - b0)
+            ip = self._eval_forward(ws, trp, tri, coef, b0, B, uid_start + b0, keep, max_nnz, words, scal)
+            ops.topk_recommend(ws.scores, B, self.I, ip if exclude_seen else None, tri if exclude_seen else None, bits, k, items[b0:],
+                               logits[b0:], probs[b0:], lse[b0:])
+        torch.cuda.synchronize()
+        return dict(items=items.cpu().numpy().astype(np.int64), probs=probs.cpu().numpy(), lse=lse.cpu().numpy())
 
 
 class Session(object):

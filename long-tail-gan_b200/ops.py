@@ -376,6 +376,17 @@ def topk_metrics(scores, n_rows, n_items, seen_ptr, seen_items, held_ptr, held_i
                                  ptr(dcg), ptr(hits), _stream()))
 
 
+def topk_recommend(scores, n_rows, n_items, seen_ptr, seen_items, allow_bits, k, out_idx, out_logit, out_prob, out_lse):
+    """Top-k eligible items per row of fp32 logits with their logits, probabilities (out_prob may be None) and the row's log-sum-exp
+    over the whole catalog. seen_ptr/seen_items (CSR, may be None) and allow_bits (the uint32 bitmap held in an int32 tensor, may be
+    None) choose what is eligible."""
+    _count(1)
+    assert scores.dtype == torch.float32 and out_idx.dtype == torch.int32
+    assert allow_bits is None or (allow_bits.dtype == torch.int32 and allow_bits.numel() >= (n_items + 31) // 32)
+    check(lib().ltg_topk_recommend(ptr(scores), scores.stride(0), n_rows, n_items, ptr(seen_ptr), ptr(seen_items), ptr(allow_bits), k,
+                                   ptr(out_idx), ptr(out_logit), ptr(out_prob), ptr(out_lse), _stream()))
+
+
 def cast_bf16(src, dst, rows, cols):
     _count(1)
     check(lib().ltg_cast_bf16(ptr(src), src.stride(0) if src.dim() > 1 else cols, ptr(dst), dst.stride(0) if dst.dim() > 1 else cols,

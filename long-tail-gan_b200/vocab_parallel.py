@@ -21,7 +21,7 @@ import torch
 import torch.distributed as dist
 
 from . import ops
-from .engine import GanEngine, TrainData, _pad, metrics_from_counts
+from .engine import GanEngine, TrainData, _pad, allow_bits, metrics_from_counts
 from .generator import H, L
 
 
@@ -59,13 +59,15 @@ def combine_softmax_stats(sa):
     return lse, sa[:, :, 1].sum(0), (sa[:, :, 2] * w).sum(0)
 
 
-def merge_topk(vals, gids, k):
+def merge_topk(vals, gids, k, with_vals=False):
     """Per-shard top-k lists side by side (vals / gids [B, R*k]: scores and GLOBAL item ids) -> the global top-k ids [B, k] ordered by
     (score desc, id asc), the tie rule of ltg_topk_metrics (eval_functions.py:17-23 leaves ties to argpartition). Two stable sorts:
-    ascending id first, then descending score."""
+    ascending id first, then descending score. with_vals: return (ids, their scores)."""
     o1 = torch.argsort(gids, dim=1, stable=True)
     vals, gids = torch.gather(vals, 1, o1), torch.gather(gids, 1, o1)
     o2 = torch.argsort(vals, dim=1, descending=True, stable=True)
+    if with_vals:
+        return torch.gather(gids, 1, o2)[:, :k], torch.gather(vals, 1, o2)[:, :k]
     return torch.gather(gids, 1, o2)[:, :k]
 
 
@@ -288,18 +290,12 @@ class CatalogShardedEngine(GanEngine):
                     sum_p=s[0][ops.S_SUM_P], sum_y=s[0][ops.S_SUM_Y])
 
     # ---- evaluation: train.py:333-348, test.py:138-173 -------------------------------------------------------------------
-    def evaluate(self, tr_indptr, tr_indices, te_indptr, te_indices, k=100, recall_ks=(20, 50), batch=None, uid_start=0, keep=None):
-        """tr_/te_ are the GLOBAL fold-in / held-out CSRs (global item ids). Every rank scores its shard, takes the exact local top-k
-        (ltg_topk_metrics, seen items masked), the k (score, global id) pairs per rank are all-gathered and merged by
-        (score desc, id asc); the metrics follow eval_functions.py:25-36,47-60 on the merged list. Returns the same dict as
-        GanEngine.evaluate on every rank."""
-        dev, v = self.device, self.vae
-        lo, I_r = self.item_lo, self.I
+    def _shard_fold_in(self, tr_indptr, tr_indices):
+        """GLOBAL fold-in CSR -> this shard's part on the device: (row pointers, shard-local item ids, 1/|x_u| over the whole row,
+        coefficient buffer, longest shard row)."""
+        dev, lo, I_r = self.device, self.item_lo, self.I
         tr_indptr = np.asarray(tr_indptr, dtype=np.int64); tr_indices = np.asarray(tr_indices, dtype=np.int64)
-        te_indptr = np.asarray(te_indptr, dtype=np.int64); te_indices = np.asarray(te_indices, dtype=np.int64)
         N = len(tr_indptr) - 1
-        batch = self.max_B if batch is None else min(batch, self.max_B)
-        keep = self.keep_vae if keep is None else keep
         deg = np.diff(tr_indptr)
         owner = np.repeat(np.arange(N, dtype=np.int64), deg)
         sel = (tr_indices >= lo) & (tr_indices < lo + I_r)
@@ -309,6 +305,49 @@ class CatalogShardedEngine(GanEngine):
         rnorm = torch.as_tensor((1.0 / np.sqrt(np.maximum(deg, 1e-12))).astype(np.float32)).to(dev)
         coef = torch.zeros(max(1, int(sel.sum())), dtype=torch.float32, device=dev)
         max_nnz = int(np.diff(lp).max()) if N > 0 else 0
+        return trp, tri, rnorm, coef, max_nnz
+
+    def _vp_eval_forward(self, fold, b0, B, uid0, keep, words, scal, scores):
+        """One batch of the inference forward over the shard (is_training = 0) into scores[:B, :I_r]: rng-step advance (snapshot in
+        words[4], the phase-A word), partial encoder gather + all-reduce, middle, fp32 decoder GEMM. `words` / `scal`: the engine's own
+        for evaluate, private copies for recommend. Returns the batch's shard-local row pointers."""
+        v = self.vae
+        trp, tri, rnorm, coef, max_nnz = fold
+        w_a = words[4:5]
+        ops.step_advance(words, scal, 0, self.lr, snap=w_a)
+        ip = trp[b0: b0 + B + 1]
+        self.pre_sum[:B].zero_()
+        ops.enc_gather_partial(ip, tri, B, self.I_global, self.item_lo, uid0, v.W_q0_b, rnorm[b0: b0 + B], keep, self.seed, 0, w_a,
+                               self.pre_sum, coef, max_nnz)
+        self._allreduce(self.pre_sum[:B])
+        ops.bias_tanh(self.pre_sum, v.view("b_q0"), B, H, self.h1)
+        ops.gemm(self.h1, v.view("W_q1", "b"), B, 2 * L, H, b_mn=True, bn=64, out_f32=self.mulv, bias=v.view("b_q1"))
+        ops.latent_fwd(self.mulv, None, B, uid0, 0.0, self.seed, 0, w_a, self.z, self.zmu, scal)
+        ops.gemm(self.z, v.view("W_p0", "b"), B, H, L, b_mn=True, bn=64, out_bf16=self.h2, bias=v.view("b_p0"), act=1)
+        ops.gemm(self.h2, v.WdT_b, B, self.I, H, bn=256, out_f32=scores, bias=v.view("b_p1"))
+        return ip
+
+    def _all_gather_cols(self, t):
+        """[B, n] on every rank -> [B, R*n], rank r's block at columns [r*n, (r+1)*n)."""
+        if self.vp_world == 1:
+            return t
+        parts = [torch.empty_like(t) for _ in range(self.vp_world)]
+        dist.all_gather(parts, t.contiguous(), group=self.group)
+        return torch.cat(parts, 1)
+
+    def evaluate(self, tr_indptr, tr_indices, te_indptr, te_indices, k=100, recall_ks=(20, 50), batch=None, uid_start=0, keep=None):
+        """tr_/te_ are the GLOBAL fold-in / held-out CSRs (global item ids). Every rank scores its shard, takes the exact local top-k
+        (ltg_topk_metrics, seen items masked), the k (score, global id) pairs per rank are all-gathered and merged by
+        (score desc, id asc); the metrics follow eval_functions.py:25-36,47-60 on the merged list. Returns the same dict as
+        GanEngine.evaluate on every rank."""
+        dev = self.device
+        lo, I_r = self.item_lo, self.I
+        te_indptr = np.asarray(te_indptr, dtype=np.int64); te_indices = np.asarray(te_indices, dtype=np.int64)
+        N = len(tr_indptr) - 1
+        batch = self.max_B if batch is None else min(batch, self.max_B)
+        keep = self.keep_vae if keep is None else keep
+        fold = self._shard_fold_in(tr_indptr, tr_indices)
+        tri = fold[1]
         scores = torch.zeros(batch, self.ld, dtype=torch.float32, device=dev)
         kk = min(k, I_r)
         idx_loc = torch.zeros(batch, kk, dtype=torch.int32, device=dev)
@@ -318,26 +357,11 @@ class CatalogShardedEngine(GanEngine):
         top_all = np.zeros((N, k), dtype=np.int64)
         for b0 in range(0, N, batch):
             B = min(batch, N - b0)
-            ops.step_advance(self.words, self.scal, 0, self.lr, snap=self.w_a)
-            ip = trp[b0: b0 + B + 1]
-            self.pre_sum[:B].zero_()
-            ops.enc_gather_partial(ip, tri, B, self.I_global, lo, uid_start + b0, v.W_q0_b, rnorm[b0: b0 + B], keep, self.seed, 0, self.w_a,
-                                   self.pre_sum, coef, max_nnz)
-            self._allreduce(self.pre_sum[:B])
-            ops.bias_tanh(self.pre_sum, v.view("b_q0"), B, H, self.h1)
-            ops.gemm(self.h1, v.view("W_q1", "b"), B, 2 * L, H, b_mn=True, bn=64, out_f32=self.mulv, bias=v.view("b_q1"))
-            ops.latent_fwd(self.mulv, None, B, uid_start + b0, 0.0, self.seed, 0, self.w_a, self.z, self.zmu, self.scal)
-            ops.gemm(self.z, v.view("W_p0", "b"), B, H, L, b_mn=True, bn=64, out_bf16=self.h2, bias=v.view("b_p0"), act=1)
-            ops.gemm(self.h2, v.WdT_b, B, I_r, H, bn=256, out_f32=scores, bias=v.view("b_p1"))
+            ip = self._vp_eval_forward(fold, b0, B, uid_start + b0, keep, self.words, self.scal, scores)
             ops.topk_metrics(scores, B, I_r, ip, tri, zero_ptr[: B + 1], one_item, kk, recall_ks, idx_loc, dcg_dummy, hits_dummy)
             val_loc = torch.gather(scores[:B, :I_r], 1, idx_loc[:B].long())
             gid_loc = idx_loc[:B].long() + lo
-            if self.vp_world > 1:
-                vals = [torch.empty_like(val_loc) for _ in range(self.vp_world)]; gids = [torch.empty_like(gid_loc) for _ in range(self.vp_world)]
-                dist.all_gather(vals, val_loc.contiguous(), group=self.group); dist.all_gather(gids, gid_loc.contiguous(), group=self.group)
-                vals, gids = torch.cat(vals, 1), torch.cat(gids, 1)
-            else:
-                vals, gids = val_loc, gid_loc
+            vals, gids = self._all_gather_cols(val_loc), self._all_gather_cols(gid_loc)
             top_all[b0: b0 + B] = merge_topk(vals, gids, k).cpu().numpy()
         # metrics on the merged lists (eval_functions.py:25-30, 47-52), fp64 like NumPy
         n_held = np.diff(te_indptr)
@@ -355,6 +379,46 @@ class CatalogShardedEngine(GanEngine):
         out = metrics_from_counts(dcg, hits, n_held, k, recall_ks)
         out["topk"] = top_all
         return out
+
+    def recommend(self, tr_indptr, tr_indices, k=100, batch=None, uid_start=0, keep=1.0, exclude_seen=True, allow=None):
+        """GanEngine.recommend over the sharded catalog, with the same GLOBAL item ids in and out; returns the same dict on every rank.
+        Every rank lists its shard's top k eligible items (ltg_topk_recommend: logits and the shard's log-sum-exp, no probabilities), the
+        (logit, global id) lists and the per-shard lse are all-gathered, the lists merged by (logit desc, id asc) and the probabilities
+        formed as exp(logit - lse) with lse = logsumexp over the shards. The engine's rng step, its phase-A snapshot and its scalars are
+        left as they were: the forward advances private copies."""
+        dev = self.device
+        lo, I_r = self.item_lo, self.I
+        N = len(tr_indptr) - 1
+        batch = self.max_B if batch is None else min(batch, self.max_B)
+        keep = self.keep_vae if keep is None else float(keep)
+        if len(tr_indices) and (np.min(tr_indices) < 0 or np.max(tr_indices) >= self.I_global):
+            raise ValueError("fold-in item ids must lie in [0, %d)" % self.I_global)
+        fold = self._shard_fold_in(tr_indptr, tr_indices)
+        tri = fold[1]
+        bits = None if allow is None else torch.from_numpy(allow_bits(allow, self.I_global, lo, lo + I_r).view(np.int32)).to(dev)
+        words, scal = self.words.clone(), self.scal.clone()
+        scores = torch.zeros(batch, self.ld, dtype=torch.float32, device=dev)
+        idx_loc = torch.empty(batch, k, dtype=torch.int32, device=dev)
+        val_loc = torch.empty(batch, k, dtype=torch.float32, device=dev)
+        lse_loc = torch.empty(batch, dtype=torch.float32, device=dev)
+        items = np.empty((N, k), dtype=np.int64)
+        probs = np.empty((N, k), dtype=np.float32)
+        lse = np.empty(N, dtype=np.float32)
+        for b0 in range(0, N, batch):
+            B = min(batch, N - b0)
+            ip = self._vp_eval_forward(fold, b0, B, uid_start + b0, keep, words, scal, scores)
+            ops.topk_recommend(scores, B, I_r, ip if exclude_seen else None, tri if exclude_seen else None, bits, k, idx_loc, val_loc, None,
+                               lse_loc)
+            il = idx_loc[:B].long()
+            gid_loc = torch.where(il >= 0, il + lo, self.I_global)   # padding sorts behind every real item of equal logit
+            vals, gids = self._all_gather_cols(val_loc[:B]), self._all_gather_cols(gid_loc)
+            lse_b = torch.logsumexp(self._all_gather_cols(lse_loc[:B, None]), dim=1)
+            top, top_val = merge_topk(vals, gids, k, with_vals=True)
+            pad = top >= self.I_global
+            items[b0: b0 + B] = torch.where(pad, -1, top).cpu().numpy()
+            probs[b0: b0 + B] = torch.where(pad, 0.0, torch.exp(top_val - lse_b[:, None])).cpu().numpy()
+            lse[b0: b0 + B] = lse_b.cpu().numpy()
+        return dict(items=items, probs=probs, lse=lse)
 
 
 def build_shard(tabs, n_items, rank, world, batch_size, vae_params=None, disc=None, seed=98765, device="cuda", first_batch=0, max_batches=None):

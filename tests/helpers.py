@@ -60,3 +60,48 @@ def dense_rows(indptr, indices, r0, r1, I):
     for r in range(r0, r1):
         X[r - r0, indices[indptr[r]:indptr[r + 1]]] = 1.0
     return X
+
+
+# ---- per-element error bounds against float64 references (torch tensors; torch is imported by the callers) -------------------------
+TAU = 2.0 ** -14      # GEMM-shaped stages: |got - ref| <= TAU * (|A| |B|) per element, fp32 accumulation of exact bf16 products
+U32 = 2.0 ** -24      # unit roundoff of fp32
+HALF_BF16 = 2.0 ** -8  # half a bf16 ulp of any value of magnitude <= x is at most 2^-8 x
+TINY = 1e-30
+
+
+def gemm_ref(A, B):
+    """float64 product of the exact (bf16 or fp32) operands and the product of their magnitudes (the per-element error scale)."""
+    A = A.double(); B = B.double()
+    return A @ B, A.abs() @ B.abs()
+
+
+def drop_last_kblock(ref, A, B):
+    """The reference with its last 64-deep k block missing: what a GEMM that skipped that block would compute."""
+    K = A.shape[1]
+    k0 = (K - 1) // 64 * 64
+    return ref - A[:, k0:].double() @ B[k0:].double()
+
+
+def assert_within(name, got, ref, bound):
+    """Every element of `got` within `bound` of the float64 `ref`; prints the worst error-to-bound ratio and returns it."""
+    import torch
+    got = got.double()
+    assert bool(torch.isfinite(got).all()), "%s: non-finite output" % name
+    err = (got - ref).abs()
+    bound = torch.broadcast_to(bound, err.shape)
+    ratio = (err / bound.clamp_min(1e-300)).max().item() if err.numel() else 0.0
+    bad = err > bound
+    if bool(bad.any()):
+        i = tuple(int(x) for x in torch.nonzero(bad)[0])
+        raise AssertionError("%s: %d of %d elements out of bound, worst err/bound %.3g; first at %s: got %r ref %r bound %r"
+                             % (name, int(bad.sum()), bad.numel(), ratio, i, got[i].item(), ref[i].item(), bound[i].item()))
+    print("[bound] %-40s worst err/bound %.3g" % (name, ratio))
+    return ratio
+
+
+def assert_detects(name, got, wrong_ref, bound):
+    """Sensitivity of a bound: a reference carrying an error of the kind that matters (a missing k block, a dropped split partial)
+    must fail it somewhere."""
+    import torch
+    err = (got.double() - wrong_ref).abs()
+    assert bool((err > torch.broadcast_to(bound, err.shape)).any()), "%s: the bound does not see the injected error" % name

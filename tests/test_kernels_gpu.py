@@ -12,6 +12,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 from oracle import ltgan_oracle as orc  # noqa: E402
 from oracle import philox  # noqa: E402
 
@@ -73,6 +74,64 @@ def test_gemm_layouts(ops, a_mn, b_mn, bn):
     assert err < 2e-2 * np.sqrt(K), err
     assert torch.isnan(out[:, N:]).all()  # nothing written outside N
     assert (outb[:, :N].float() - ref).abs().max().item() < 0.02 * ref.abs().max().item() + 0.1
+    for Me, Ke in GEMM_EDGE_CASES:
+        _gemm_edge_case(ops, Me, 264, Ke, bn, a_mn, b_mn)
+
+
+# (M, K): M sets the cluster size of launch_gemm (1, 2, 4 for 1, 2, 3-4 row blocks; 2 beyond), the K values the tails
+GEMM_EDGE_CASES = [(100, 52),    # cluster 1
+                   (200, 4100),  # cluster 2
+                   (300, 1),     # cluster 4 with a zero-filled padding row block, K = 1 (a one-user batch's weight gradient)
+                   (500, 500),   # cluster 4
+                   (600, 52),    # cluster 2 with a padding block (dW_q1)
+                   (1300, 500)]  # cluster 2, six groups, the last with a padding block
+
+
+def _gemm_edge_case(ops, M, N, K, bn, a_mn, b_mn):
+    """One GEMM shape through every epilogue path that stores fp32, per element against float64 (tests/helpers.py): plain store with
+    the aux column diverted, split-K partials at split_stride with more splits than k blocks (the empty partials must store zeros, not
+    leave the NaN they were filled with), split-K with atomics. Operand pitch padding holds NaN: TMA must never read it."""
+    from helpers import TAU, TINY, gemm_ref, drop_last_kblock, assert_within, assert_detects
+    g = torch.Generator(device="cuda").manual_seed(M * 7 + K + bn)
+    A = torch.randn(M, K, device="cuda", generator=g).bfloat16()
+    Bm = torch.randn(N, K, device="cuda", generator=g).bfloat16()
+
+    def stored(X, mn):
+        rows, cols = (X.shape[1], X.shape[0]) if mn else X.shape
+        P = torch.full((rows, (cols + 7) // 8 * 8 + 8), float("nan"), device="cuda", dtype=torch.bfloat16)
+        P[:, :cols] = X.t() if mn else X
+        return P
+    Ap, Bp = stored(A, a_mn), stored(Bm, b_mn)
+    ref, mag = gemm_ref(A, Bm.t())
+    bound = TAU * mag + TINY
+    tag = "gemm M=%d N=%d K=%d bn=%d a_mn=%d b_mn=%d" % (M, N, K, bn, a_mn, b_mn)
+    out = torch.full((M, N + 8), float("nan"), device="cuda")
+    aux = torch.full((M,), float("nan"), device="cuda")
+    ops.gemm(Ap, Bp, M, N, K, a_mn=a_mn, b_mn=b_mn, bn=bn, out_f32=out, aux_col=N - 1, aux_out=aux)
+    kb = (K + 63) // 64
+    splits = kb + 2
+    parts = torch.full((splits, M, N + 8), float("nan"), device="cuda")
+    ops.gemm(Ap, Bp, M, N, K, a_mn=a_mn, b_mn=b_mn, bn=bn, splits=splits, out_f32=parts, ld_f32=N + 8, split_stride=M * (N + 8))
+    acc = torch.zeros(M, N + 8, device="cuda")
+    ops.gemm(Ap, Bp, M, N, K, a_mn=a_mn, b_mn=b_mn, bn=bn, splits=3, atomic=True, out_f32=acc)
+    torch.cuda.synchronize()
+    assert_within(tag, out[:, :N - 1], ref[:, :N - 1], bound[:, :N - 1])
+    assert_detects(tag + " minus last k block", out[:, :N - 1], drop_last_kblock(ref, A, Bm.t())[:, :N - 1], bound[:, :N - 1])
+    assert_within(tag + " aux column", aux, ref[:, N - 1], bound[:, N - 1])
+    assert torch.isnan(out[:, N - 1:]).all()   # the aux column and the pitch padding are not written
+    per = (kb + splits - 1) // splits
+    used = [s for s in range(splits) if s * per < kb]
+    assert len(used) < splits
+    for s in range(splits):
+        if s not in used:
+            assert (parts[s, :, :N] == 0).all(), "%s: empty split %d must store zeros" % (tag, s)
+    assert torch.isnan(parts[:, :, N:]).all()
+    got = parts[:, :, :N].double().sum(0)
+    assert_within(tag + " split_stride", got, ref, bound)
+    if len(used) > 1:
+        assert_detects(tag + " without its last partial", got - parts[used[-1], :, :N].double(), ref, bound)
+    assert_within(tag + " atomic split-K", acc[:, :N], ref, bound)
+    assert (acc[:, N:] == 0).all()
 
 
 def test_gemm_splitk_bias_act_aux(ops):

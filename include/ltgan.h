@@ -307,6 +307,18 @@ int ltg_disc_head(const void* Y3_bf16, int ld, int P, int h3, const float* w4, c
 int ltg_topk_metrics(const void* scores, int is_bf16, int64_t ld, int n_rows, int n_items,
                      const int32_t* seen_ptr, const int32_t* seen_items, const int32_t* held_ptr, const int32_t* held_items,
                      int k, const int32_t* rk_host, int n_rk, int32_t* topk_idx, double* dcg, int32_t* hits, void* stream);
+/* Long-tail evaluation: ltg_topk_metrics (same arguments, same lists, bit-identical topk_idx / dcg / hits, same staged / streaming
+ * choice) plus, per row, from the same sorted list of kk = min(k, n_items) items: dcg_niche[n] (fp64) = sum over listed held-out NICHE
+ * items of 1/log2(r+2), hits_niche[n, n_rk] = |top-rk[j] AND heldout AND niche|, n_niche_top[n] = |list AND niche|, pop_sum[n] = sum of
+ * item_pop over the list. niche_bits: (n_items+31)/32 words, bit i%32 of word i/32 set for a niche item (the allow_bits format of
+ * ltg_topk_recommend); item_pop [n_items]: training interactions per item. rec_count [n_items] += 1 for every listed item of every row
+ * with a non-empty held-out set: it is NOT cleared, so it accumulates across launches (zero it before the first). Every pointer is
+ * required except seen_ptr / seen_items and topk_idx (may be NULL, as for ltg_topk_metrics) and rk_host / hits when n_rk == 0.       */
+int ltg_topk_longtail(const void* scores, int is_bf16, int64_t ld, int n_rows, int n_items,
+                      const int32_t* seen_ptr, const int32_t* seen_items, const int32_t* held_ptr, const int32_t* held_items,
+                      int k, const int32_t* rk_host, int n_rk, int32_t* topk_idx, double* dcg, int32_t* hits,
+                      const uint32_t* niche_bits, const int32_t* item_pop, double* dcg_niche, int32_t* hits_niche, int32_t* n_niche_top,
+                      int64_t* pop_sum, int32_t* rec_count, void* stream);
 /* Recommendation lists. Per row u of fp32 logits (pitch ld; columns n_items..ld are never read), an item is ELIGIBLE when it is not in
  * seen_items[seen_ptr[u] .. seen_ptr[u+1]) and its bit of allow_bits ((n_items+31)/32 words, bit i%32 of word i/32) is set. Excluded
  * items are never listed. out_idx [n, k]: the min(k, #eligible) eligible items with the highest logits ordered by (logit desc, item id

@@ -145,6 +145,7 @@ SIGNATURES = {
     "ltg_disc_fused_set_trace": (_I, [_P]),
     "ltg_disc_head": (_I, [_P, _I, _I, _I, _P, _P, _P, _F, _P, _P, _P, _P, _P, _P]),
     "ltg_topk_metrics": (_I, [_P, _I, _I64, _I, _I, _P, _P, _P, _P, _I, _P, _I, _P, _P, _P, _P]),
+    "ltg_topk_longtail": (_I, [_P, _I, _I64, _I, _I, _P, _P, _P, _P, _I, _P, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "ltg_topk_recommend": (_I, [_P, _I64, _I, _I, _P, _P, _P, _I, _P, _P, _P, _P, _P]),
     "ltg_cast_bf16": (_I, [_P, _I64, _P, _I64, _I64, _I64, _P]),
     "ltg_csv_open": (_I, [_P, _P, _P, _I, _P, _P]),

@@ -64,12 +64,60 @@ __device__ uint32_t radix_select_desc(int n, uint32_t k, ValFn val, uint32_t* s_
   return prefix;
 }
 
-template <bool BF16>
+// Long-tail outputs of ltg_topk_longtail (the LT = true instantiations of the two metrics kernels below).
+struct LtArgs {
+  const uint32_t* niche_bits;   // [(n_items+31)/32]: bit i%32 of word i/32 set when item i is a niche item
+  const int32_t* item_pop;      // [n_items]: training interactions per item
+  double* dcg_niche;            // [n_rows]
+  int32_t* hits_niche;          // [n_rows, n_rk]
+  int32_t* n_niche_top;         // [n_rows]
+  long long* pop_sum;           // [n_rows]
+  int32_t* rec_count;           // [n_items], accumulated across launches
+};
+
+// Called by every thread of the CTA once the row's list is sorted: thread tid < kk holds list entry tid (item idx, held-out hit `hit`).
+// Niche DCG uses the same terms and the same warp / cross-warp summation order as dcg. The niche bits and popularities are read through
+// the read-only path: n_items / 8 bytes of bitmap and 4 * n_items bytes of counts are shared by every row and stay in L2.
+__device__ __forceinline__ void longtail_row(const LtArgs& a, int u, int kk, int idx, bool hit, bool has_held, int4 rk, int n_rk) {
+  __shared__ double s_ndcg[TK_MAXK / 32];
+  __shared__ long long s_pop[TK_MAXK / 32];
+  __shared__ int s_cnt[TK_MAXK / 32][5];   // per warp: niche hits at rk.x .. rk.w, niche items listed
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  bool niche = false;
+  long long pop = 0;
+  if (tid < kk) {
+    niche = (__ldg(a.niche_bits + (idx >> 5)) >> (idx & 31)) & 1u;
+    pop = __ldg(a.item_pop + idx);
+    if (has_held) atomicAdd(a.rec_count + idx, 1);
+  }
+  if (tid < TK_MAXK) {   // whole warps: TK_MAXK is a multiple of 32
+    const bool nh = hit && niche;
+    const double term = warp_sum_d(nh ? 1.0 / log2((double)(tid + 2)) : 0.0);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) pop += __shfl_xor_sync(0xffffffffu, pop, o);
+    const int c0 = __popc(__ballot_sync(0xffffffffu, nh && tid < rk.x)), c1 = __popc(__ballot_sync(0xffffffffu, nh && tid < rk.y));
+    const int c2 = __popc(__ballot_sync(0xffffffffu, nh && tid < rk.z)), c3 = __popc(__ballot_sync(0xffffffffu, nh && tid < rk.w));
+    const int cn = __popc(__ballot_sync(0xffffffffu, niche));
+    if (lane == 0) {
+      s_ndcg[warp] = term; s_pop[warp] = pop;
+      s_cnt[warp][0] = c0; s_cnt[warp][1] = c1; s_cnt[warp][2] = c2; s_cnt[warp][3] = c3; s_cnt[warp][4] = cn;
+    }
+  }
+  __syncthreads();
+  if (tid == 0) {
+    a.dcg_niche[u] = s_ndcg[0] + s_ndcg[1] + s_ndcg[2] + s_ndcg[3];
+    a.pop_sum[u] = s_pop[0] + s_pop[1] + s_pop[2] + s_pop[3];
+    a.n_niche_top[u] = s_cnt[0][4] + s_cnt[1][4] + s_cnt[2][4] + s_cnt[3][4];
+    for (int j = 0; j < n_rk; ++j) a.hits_niche[(size_t)u * n_rk + j] = s_cnt[0][j] + s_cnt[1][j] + s_cnt[2][j] + s_cnt[3][j];
+  }
+}
+
+template <bool BF16, bool LT>
 __global__ void __launch_bounds__(TK_THREADS)
 topk_metrics_kernel(const void* __restrict__ scores, int64_t ld, int n_items,
                     const int32_t* __restrict__ seen_ptr, const int32_t* __restrict__ seen_items,
                     const int32_t* __restrict__ held_ptr, const int32_t* __restrict__ held_items,
-                    int k, int4 rk, int n_rk, int32_t* __restrict__ topk_idx, double* __restrict__ dcg, int32_t* __restrict__ hits) {
+                    int k, int4 rk, int n_rk, int32_t* __restrict__ topk_idx, double* __restrict__ dcg, int32_t* __restrict__ hits, LtArgs lt) {
   extern __shared__ uint32_t s_bitmap[];  // [(n_items+31)/32]
   __shared__ uint32_t s_hist[256];
   __shared__ uint32_t s_sel[3];
@@ -133,6 +181,8 @@ topk_metrics_kernel(const void* __restrict__ scores, int64_t ld, int n_items,
   }
   // metrics
   double term = 0.0;
+  int lt_idx = 0;
+  bool lt_hit = false;
   if (tid < kk) {
     const int idx = (int)(~(uint32_t)(s_win[tid] & 0xFFFFFFFFull));
     if (topk_idx != nullptr) topk_idx[(size_t)u * k + tid] = idx;
@@ -151,6 +201,7 @@ topk_metrics_kernel(const void* __restrict__ scores, int64_t ld, int n_items,
       if (n_rk > 2 && tid < rk.z) atomicAdd(&s_hits[2], 1);
       if (n_rk > 3 && tid < rk.w) atomicAdd(&s_hits[3], 1);
     }
+    if constexpr (LT) { lt_idx = idx; lt_hit = hit; }
   } else if (tid < k && topk_idx != nullptr) {
     topk_idx[(size_t)u * k + tid] = -1;
   }
@@ -163,6 +214,7 @@ topk_metrics_kernel(const void* __restrict__ scores, int64_t ld, int n_items,
     dcg[u] = s_dcg[0] + s_dcg[1] + s_dcg[2] + s_dcg[3];
     for (int j = 0; j < n_rk; ++j) hits[(size_t)u * n_rk + j] = s_hits[j];
   }
+  if constexpr (LT) longtail_row(lt, u, kk, lt_idx, lt_hit, held_ptr[u + 1] > held_ptr[u], rk, n_rk);
 }
 
 
@@ -241,13 +293,13 @@ __device__ uint32_t radix_select11(int n, uint32_t k, ValFn val, uint32_t* s_his
   return prefix;
 }
 
-template <bool BF16>
+template <bool BF16, bool LT>
 __global__ void __launch_bounds__(TS_THREADS)
 topk_staged_kernel(const void* __restrict__ scores, int64_t ld, int n_items,
                    const int32_t* __restrict__ seen_ptr, const int32_t* __restrict__ seen_items,
                    const int32_t* __restrict__ held_ptr, const int32_t* __restrict__ held_items,
                    int k, int4 rk, int n_rk, int32_t* __restrict__ topk_idx, double* __restrict__ dcg, int32_t* __restrict__ hits,
-                   bool use_prefilter) {
+                   bool use_prefilter, LtArgs lt) {
   extern __shared__ __align__(16) uint32_t s_keys[];   // [n_items rounded up to 8]
   __shared__ __align__(16) uint32_t s_hist[TS_BINS];
   __shared__ uint32_t s_warp[TS_THREADS / 32];
@@ -374,6 +426,8 @@ topk_staged_kernel(const void* __restrict__ scores, int64_t ld, int n_items,
   }
   // metrics (eval_functions.py:25-30, 47-52)
   double term = 0.0;
+  int lt_idx = 0;
+  bool lt_hit = false;
   if (tid < kk) {
     const int idx = (int)(~(uint32_t)(s_win[tid] & 0xFFFFFFFFull));
     if (topk_idx != nullptr) topk_idx[(size_t)u * k + tid] = idx;
@@ -392,6 +446,7 @@ topk_staged_kernel(const void* __restrict__ scores, int64_t ld, int n_items,
       if (n_rk > 2 && tid < rk.z) atomicAdd(&s_hits[2], 1);
       if (n_rk > 3 && tid < rk.w) atomicAdd(&s_hits[3], 1);
     }
+    if constexpr (LT) { lt_idx = idx; lt_hit = hit; }
   } else if (tid < k && topk_idx != nullptr) {
     topk_idx[(size_t)u * k + tid] = -1;
   }
@@ -404,13 +459,19 @@ topk_staged_kernel(const void* __restrict__ scores, int64_t ld, int n_items,
     dcg[u] = s_dcg[0] + s_dcg[1] + s_dcg[2] + s_dcg[3];
     for (int j = 0; j < n_rk; ++j) hits[(size_t)u * n_rk + j] = s_hits[j];
   }
+  if constexpr (LT) longtail_row(lt, u, kk, lt_idx, lt_hit, held_ptr[u + 1] > held_ptr[u], rk, n_rk);
 }
 
 }  // namespace
 
-extern "C" int ltg_topk_metrics(const void* scores, int is_bf16, int64_t ld, int n_rows, int n_items,
-                                const int32_t* seen_ptr, const int32_t* seen_items, const int32_t* held_ptr, const int32_t* held_items,
-                                int k, const int32_t* rk_host, int n_rk, int32_t* topk_idx, double* dcg, int32_t* hits, void* stream) {
+namespace {
+
+// The host side of ltg_topk_metrics and ltg_topk_longtail: argument checks, then the staged or the streaming kernel, chosen the same
+// way for both (LT only adds the long-tail outputs).
+template <bool LT>
+int topk_metrics_launch(const void* scores, int is_bf16, int64_t ld, int n_rows, int n_items, const int32_t* seen_ptr, const int32_t* seen_items,
+                        const int32_t* held_ptr, const int32_t* held_items, int k, const int32_t* rk_host, int n_rk, int32_t* topk_idx, double* dcg,
+                        int32_t* hits, const LtArgs& lt, void* stream) {
   LTG_REQUIRE(scores && held_ptr && held_items && dcg);
   LTG_REQUIRE(k >= 1 && k <= TK_MAXK && n_rk >= 0 && n_rk <= 4 && (n_rk == 0 || (rk_host != nullptr && hits != nullptr)));
   LTG_REQUIRE(seen_ptr == nullptr || seen_items != nullptr);
@@ -428,17 +489,17 @@ extern "C" int ltg_topk_metrics(const void* scores, int is_bf16, int64_t ld, int
     static int prefilter = -1;   // LTG_TOPK_PREFILTER=0: select over the whole row (A/B switch)
     if (prefilter < 0) { const char* e = getenv("LTG_TOPK_PREFILTER"); prefilter = (e != nullptr && e[0] == '0') ? 0 : 1; }
     if (sm > opted_s[is_bf16 ? 1 : 0]) {
-      cudaError_t e = is_bf16 ? cudaFuncSetAttribute(topk_staged_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm)
-                              : cudaFuncSetAttribute(topk_staged_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+      cudaError_t e = is_bf16 ? cudaFuncSetAttribute(topk_staged_kernel<true, LT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm)
+                              : cudaFuncSetAttribute(topk_staged_kernel<false, LT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
       if (e != cudaSuccess) { ltg_set_last_error(cudaGetErrorString(e), __FILE__, __LINE__); return LTG_ERR_CUDA; }
       opted_s[is_bf16 ? 1 : 0] = sm;
     }
     if (is_bf16)
-      topk_staged_kernel<true><<<n_rows, TS_THREADS, sm, (cudaStream_t)stream>>>(scores, ld, n_items, seen_ptr, seen_items, held_ptr, held_items, k, rk,
-                                                                                 n_rk, topk_idx, dcg, hits, prefilter != 0);
+      topk_staged_kernel<true, LT><<<n_rows, TS_THREADS, sm, (cudaStream_t)stream>>>(scores, ld, n_items, seen_ptr, seen_items, held_ptr, held_items, k,
+                                                                                     rk, n_rk, topk_idx, dcg, hits, prefilter != 0, lt);
     else
-      topk_staged_kernel<false><<<n_rows, TS_THREADS, sm, (cudaStream_t)stream>>>(scores, ld, n_items, seen_ptr, seen_items, held_ptr, held_items, k, rk,
-                                                                                  n_rk, topk_idx, dcg, hits, prefilter != 0);
+      topk_staged_kernel<false, LT><<<n_rows, TS_THREADS, sm, (cudaStream_t)stream>>>(scores, ld, n_items, seen_ptr, seen_items, held_ptr, held_items,
+                                                                                      k, rk, n_rk, topk_idx, dcg, hits, prefilter != 0, lt);
     LTG_CHECK_LAUNCH();
     return LTG_OK;
   }
@@ -446,19 +507,39 @@ extern "C" int ltg_topk_metrics(const void* scores, int is_bf16, int64_t ld, int
   LTG_REQUIRE(smem <= 200 * 1024);
   static size_t opted[2] = {40 * 1024, 40 * 1024};
   if (smem > opted[is_bf16 ? 1 : 0]) {
-    cudaError_t e = is_bf16 ? cudaFuncSetAttribute(topk_metrics_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
-                            : cudaFuncSetAttribute(topk_metrics_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = is_bf16 ? cudaFuncSetAttribute(topk_metrics_kernel<true, LT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
+                            : cudaFuncSetAttribute(topk_metrics_kernel<false, LT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) { ltg_set_last_error(cudaGetErrorString(e), __FILE__, __LINE__); return LTG_ERR_CUDA; }
     opted[is_bf16 ? 1 : 0] = smem;
   }
   if (is_bf16)
-    topk_metrics_kernel<true><<<n_rows, TK_THREADS, smem, (cudaStream_t)stream>>>(scores, ld, n_items, seen_ptr, seen_items, held_ptr, held_items, k,
-                                                                                 rk, n_rk, topk_idx, dcg, hits);
+    topk_metrics_kernel<true, LT><<<n_rows, TK_THREADS, smem, (cudaStream_t)stream>>>(scores, ld, n_items, seen_ptr, seen_items, held_ptr, held_items,
+                                                                                     k, rk, n_rk, topk_idx, dcg, hits, lt);
   else
-    topk_metrics_kernel<false><<<n_rows, TK_THREADS, smem, (cudaStream_t)stream>>>(scores, ld, n_items, seen_ptr, seen_items, held_ptr, held_items, k,
-                                                                                  rk, n_rk, topk_idx, dcg, hits);
+    topk_metrics_kernel<false, LT><<<n_rows, TK_THREADS, smem, (cudaStream_t)stream>>>(scores, ld, n_items, seen_ptr, seen_items, held_ptr, held_items,
+                                                                                      k, rk, n_rk, topk_idx, dcg, hits, lt);
   LTG_CHECK_LAUNCH();
   return LTG_OK;
+}
+
+}  // namespace
+
+extern "C" int ltg_topk_metrics(const void* scores, int is_bf16, int64_t ld, int n_rows, int n_items,
+                                const int32_t* seen_ptr, const int32_t* seen_items, const int32_t* held_ptr, const int32_t* held_items,
+                                int k, const int32_t* rk_host, int n_rk, int32_t* topk_idx, double* dcg, int32_t* hits, void* stream) {
+  return topk_metrics_launch<false>(scores, is_bf16, ld, n_rows, n_items, seen_ptr, seen_items, held_ptr, held_items, k, rk_host, n_rk, topk_idx,
+                                    dcg, hits, LtArgs{}, stream);
+}
+
+extern "C" int ltg_topk_longtail(const void* scores, int is_bf16, int64_t ld, int n_rows, int n_items,
+                                 const int32_t* seen_ptr, const int32_t* seen_items, const int32_t* held_ptr, const int32_t* held_items,
+                                 int k, const int32_t* rk_host, int n_rk, int32_t* topk_idx, double* dcg, int32_t* hits,
+                                 const uint32_t* niche_bits, const int32_t* item_pop, double* dcg_niche, int32_t* hits_niche, int32_t* n_niche_top,
+                                 int64_t* pop_sum, int32_t* rec_count, void* stream) {
+  LTG_REQUIRE(niche_bits && item_pop && dcg_niche && hits_niche && n_niche_top && pop_sum && rec_count);
+  const LtArgs lt{niche_bits, item_pop, dcg_niche, hits_niche, n_niche_top, reinterpret_cast<long long*>(pop_sum), rec_count};
+  return topk_metrics_launch<true>(scores, is_bf16, ld, n_rows, n_items, seen_ptr, seen_items, held_ptr, held_items, k, rk_host, n_rk, topk_idx,
+                                   dcg, hits, lt, stream);
 }
 
 

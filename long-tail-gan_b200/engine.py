@@ -1142,9 +1142,17 @@ class GanEngine(object):
         ops.gemm(ws.h2, v.WdT_b, B, self.I, H, bn=256, out_f32=ws.scores, bias=v.view("b_p1"))
         return ip
 
-    def evaluate(self, tr_indptr, tr_indices, te_indptr, te_indices, k=100, recall_ks=(20, 50), batch=None, uid_start=0, keep=None):
+    def evaluate(self, tr_indptr, tr_indices, te_indptr, te_indices, k=100, recall_ks=(20, 50), batch=None, uid_start=0, keep=None,
+                 niche=None, item_pop=None):
         """Scores every eval user from its fold-in interactions, masks them, ranks, and returns the per-user lists
-        (ndcg@k, recall@rk...) over users with a non-empty held-out set, exactly like eval_functions.py."""
+        (ndcg@k, recall@rk...) over users with a non-empty held-out set, exactly like eval_functions.py.
+
+        niche (optional): niche item ids or a boolean mask of length I; item_pop (required with niche): int array [I] of training
+        interactions per item. With them every batch ranks through ltg_topk_longtail instead of ltg_topk_metrics (same lists, same
+        values for the keys above) and the result also holds the long-tail keys of longtail_from_counts."""
+        lt = niche is not None or item_pop is not None
+        if lt:
+            niche_mask, item_pop = longtail_inputs(niche, item_pop, self.I)
         dev = self.device
         N = len(tr_indptr) - 1
         batch = self._eval_batch(N, batch)
@@ -1182,6 +1190,14 @@ class GanEngine(object):
                 state["tei"] = torch.as_tensor(np.ascontiguousarray(te_indices if len(te_indices) else np.zeros(1), dtype=np.int32)).to(dev, non_blocking=True)
                 state["dcg"] = torch.zeros(N, dtype=torch.float64, device=dev)
                 state["hits"] = torch.zeros(N, max(1, len(recall_ks)), dtype=torch.int32, device=dev)
+                if lt:
+                    state["bits"] = torch.from_numpy(allow_bits(niche_mask, self.I).view(np.int32)).to(dev, non_blocking=True)
+                    state["pop"] = torch.from_numpy(item_pop.astype(np.int32)).to(dev, non_blocking=True)
+                    state["dcg_niche"] = torch.empty(N, dtype=torch.float64, device=dev)
+                    state["hits_niche"] = torch.empty(N, max(1, len(recall_ks)), dtype=torch.int32, device=dev)
+                    state["n_niche_top"] = torch.empty(N, dtype=torch.int32, device=dev)
+                    state["pop_sum"] = torch.empty(N, dtype=torch.int64, device=dev)
+                    state["rec_count"] = torch.zeros(self.I, dtype=torch.int32, device=dev)
             main.wait_stream(up)
 
         for b0 in range(0, N, batch):
@@ -1190,13 +1206,28 @@ class GanEngine(object):
             ip = self._eval_forward(ws, trp, tri, coef, b0, B, uid_start + b0, keep, max_eval_nnz, self.words, self.scal)
             if b0 == 0:
                 upload_rest()
-            ops.topk_metrics(scores, B, self.I, ip, tri, state["tep"][b0: b0 + B + 1], state["tei"], k, recall_ks, None, state["dcg"][b0:],
-                             state["hits"][b0:])
+            if lt:
+                ops.topk_longtail(scores, B, self.I, ip, tri, state["tep"][b0: b0 + B + 1], state["tei"], k, recall_ks, None, state["dcg"][b0:],
+                                  state["hits"][b0:], state["bits"], state["pop"], state["dcg_niche"][b0:], state["hits_niche"][b0:],
+                                  state["n_niche_top"][b0:], state["pop_sum"][b0:], state["rec_count"])
+            else:
+                ops.topk_metrics(scores, B, self.I, ip, tri, state["tep"][b0: b0 + B + 1], state["tei"], k, recall_ks, None, state["dcg"][b0:],
+                                 state["hits"][b0:])
         if N <= 0:
             upload_rest()
+        if lt:   # |H_u & N| per row, counted while the GPU ranks
+            te_ptr = np.asarray(te_indptr, dtype=np.int64)
+            csum_niche = np.concatenate([[0], np.cumsum(niche_mask[np.asarray(te_indices, dtype=np.int64)], dtype=np.int64)])
+            n_held_niche = csum_niche[te_ptr[1:]] - csum_niche[te_ptr[:-1]]
         dcg, hits = state["dcg"], state["hits"][:, :len(recall_ks)]
         torch.cuda.synchronize()
-        return metrics_from_counts(dcg.cpu().numpy(), hits.cpu().numpy(), np.diff(np.asarray(te_indptr, dtype=np.int64)), k, recall_ks)
+        n_held = np.diff(np.asarray(te_indptr, dtype=np.int64))
+        out = metrics_from_counts(dcg.cpu().numpy(), hits.cpu().numpy(), n_held, k, recall_ks)
+        if lt:
+            out.update(longtail_from_counts(state["dcg_niche"].cpu().numpy(), state["hits_niche"][:, :len(recall_ks)].cpu().numpy(),
+                                            state["n_niche_top"].cpu().numpy(), state["pop_sum"].cpu().numpy(), state["rec_count"].cpu().numpy(),
+                                            n_held, n_held_niche, niche_mask, k, recall_ks))
+        return out
 
     def recommend(self, tr_indptr, tr_indices, k=100, batch=None, uid_start=0, keep=1.0, exclude_seen=True, allow=None):
         """Top-k recommendation lists for the users whose fold-in interactions are the CSR rows (tr_indptr, tr_indices). Users are scored
@@ -1301,4 +1332,67 @@ def metrics_from_counts(dcg, hits, n_held, k, recall_ks):
     for j, rk in enumerate(recall_ks):
         denom = np.minimum(rk, n_held)
         out["recall@%d" % rk] = (hits[keep, j].astype(np.float32) / denom[keep]).tolist()
+    return out
+
+
+def longtail_inputs(niche, item_pop, n_items):
+    """Validates evaluate's niche / item_pop arguments -> (niche mask bool [n_items], item_pop int64 [n_items])."""
+    if niche is None or item_pop is None:
+        raise ValueError("long-tail evaluation needs both niche and item_pop")
+    mask = allow_mask(niche, n_items)
+    if not mask.any():
+        raise ValueError("the niche set is empty")
+    pop = np.asarray(item_pop)
+    if pop.shape != (n_items,):
+        raise ValueError("item_pop must have shape (%d,), got %s" % (n_items, pop.shape))
+    if not (np.issubdtype(pop.dtype, np.integer) or pop.dtype == bool):
+        raise ValueError("item_pop must hold integer counts, got dtype %s" % pop.dtype)
+    pop = pop.astype(np.int64)
+    if n_items and (pop.min() < 0 or pop.max() > np.iinfo(np.int32).max):
+        raise ValueError("item_pop counts must lie in [0, 2**31)")
+    return mask, pop
+
+
+def longtail_from_counts(dcg_niche, hits_niche, n_niche_top, pop_sum, rec_count, n_held, n_held_niche, niche_mask, k, recall_ks):
+    """Host tail of long-tail evaluation, float64. Per user u with list L_u (kk = min(k, I) items) and held-out set H_u, N the niche set:
+      niche_ndcg@k      dcg_niche / IDCG(min(|H_u & N|, k))           over users with |H_u & N| > 0, in row order
+      niche_recall@rk   hits_niche[:, j] / min(rk, |H_u & N|)         same users
+      niche_share@k     |L_u & N| / kk                                  over users with |H_u| > 0 (the users of ndcg@k)
+      avg_pop@k         sum of item_pop over L_u / kk                   same users
+    and over the lists of the users with |H_u| > 0, c = rec_count (how many of those lists hold each item):
+      coverage@k        #{i : c[i] > 0} / I
+      niche_coverage@k  #{i in N : c[i] > 0} / |N|
+      gini@k            sum_j (2j - I - 1) c_(j) / (I sum c), c_(j) ascending, j = 1..I; 0 when sum c = 0."""
+    n_held = np.asarray(n_held, dtype=np.int64)
+    n_held_niche = np.asarray(n_held_niche, dtype=np.int64)
+    niche_mask = np.asarray(niche_mask, dtype=bool)
+    c = np.asarray(rec_count, dtype=np.int64)
+    I = len(niche_mask)
+    kk = min(k, I)
+    tp = 1.0 / np.log2(np.arange(2, k + 2))
+    csum = np.concatenate([[0.0], np.cumsum(tp)])
+    has_niche = n_held_niche > 0
+    out = {"niche_ndcg@%d" % k: (np.asarray(dcg_niche, dtype=np.float64)[has_niche] / csum[np.minimum(n_held_niche, k)][has_niche]).tolist()}
+    hits_niche = np.asarray(hits_niche).reshape(len(n_held), -1)
+    for j, rk in enumerate(recall_ks):
+        out["niche_recall@%d" % rk] = (hits_niche[has_niche, j].astype(np.float64) / np.minimum(rk, n_held_niche[has_niche])).tolist()
+    keep = n_held > 0
+    out["niche_share@%d" % k] = (np.asarray(n_niche_top, dtype=np.float64)[keep] / kk).tolist()
+    out["avg_pop@%d" % k] = (np.asarray(pop_sum, dtype=np.float64)[keep] / kk).tolist()
+    out["coverage@%d" % k] = float(np.count_nonzero(c)) / I
+    out["niche_coverage@%d" % k] = float(np.count_nonzero(c[niche_mask])) / int(niche_mask.sum())
+    total = int(c.sum())
+    weights = 2 * np.arange(1, I + 1, dtype=np.int64) - I - 1
+    out["gini@%d" % k] = float(int(np.dot(weights, np.sort(c)))) / float(I * total) if total > 0 else 0.0
+    return out
+
+
+def longtail_summary(m, k=100, recall_ks=(20, 50)):
+    """The eight long-tail numbers of an evaluate result that train.py records and `test.py --long-tail` prints, in that order: niche
+    NDCG, niche recall per cut-off (per-user lists averaged), niche share, average popularity, coverage, niche coverage and Gini."""
+    out = {"niche_ndcg": float(np.mean(m["niche_ndcg@%d" % k]))}
+    for rk in recall_ks:
+        out["niche_r%d" % rk] = float(np.mean(m["niche_recall@%d" % rk]))
+    out.update(niche_share=float(np.mean(m["niche_share@%d" % k])), avg_pop=float(np.mean(m["avg_pop@%d" % k])),
+               coverage=m["coverage@%d" % k], niche_coverage=m["niche_coverage@%d" % k], gini=m["gini@%d" % k])
     return out

@@ -376,6 +376,25 @@ def topk_metrics(scores, n_rows, n_items, seen_ptr, seen_items, held_ptr, held_i
                                  ptr(dcg), ptr(hits), _stream()))
 
 
+def topk_longtail(scores, n_rows, n_items, seen_ptr, seen_items, held_ptr, held_items, k, rks, topk_idx, dcg, hits, niche_bits, item_pop,
+                  dcg_niche, hits_niche, n_niche_top, pop_sum, rec_count):
+    """topk_metrics plus the long-tail counts of the same lists: niche DCG, niche hits per recall cut-off, niche items listed and the
+    popularity sum per row; rec_count [n_items] (int32, not cleared) += one per listed item of every row with held-out items.
+    niche_bits is the allow_bits bitmap held in an int32 tensor."""
+    _count(1)
+    import numpy as np
+    rk = np.asarray(list(rks), dtype=np.int32)
+    is_bf16 = scores.dtype == torch.bfloat16
+    assert niche_bits.dtype == torch.int32 and niche_bits.numel() >= (n_items + 31) // 32
+    assert item_pop.dtype == torch.int32 and item_pop.numel() >= n_items and rec_count.dtype == torch.int32 and rec_count.numel() >= n_items
+    assert dcg_niche.dtype == torch.float64 and hits_niche.dtype == torch.int32 and n_niche_top.dtype == torch.int32
+    assert pop_sum.dtype == torch.int64
+    check(lib().ltg_topk_longtail(ptr(scores), int(is_bf16), scores.stride(0), n_rows, n_items, ptr(seen_ptr), ptr(seen_items),
+                                  ptr(held_ptr), ptr(held_items), k, rk.ctypes.data if len(rk) else None, len(rk), ptr(topk_idx),
+                                  ptr(dcg), ptr(hits), ptr(niche_bits), ptr(item_pop), ptr(dcg_niche), ptr(hits_niche), ptr(n_niche_top),
+                                  ptr(pop_sum), ptr(rec_count), _stream()))
+
+
 def topk_recommend(scores, n_rows, n_items, seen_ptr, seen_items, allow_bits, k, out_idx, out_logit, out_prob, out_lse):
     """Top-k eligible items per row of fp32 logits with their logits, probabilities (out_prob may be None) and the row's log-sum-exp
     over the whole catalog. seen_ptr/seen_items (CSR, may be None) and allow_bits (the uint32 bitmap held in an int32 tensor, may be

@@ -23,7 +23,7 @@ if __package__ in (None, ""):
 from . import data_processing as dp                      # noqa: E402
 from .data_processing import load_item_one_hot_features as load_item_features  # noqa: E402,F401
 from .discriminator import discriminator                 # noqa: E402
-from .engine import GanEngine, TrainData                 # noqa: E402
+from .engine import GanEngine, TrainData, longtail_summary   # noqa: E402
 from .generator import generator_VAECF as generator      # noqa: E402
 from .generator import MultiVAE                          # noqa: E402
 from .dist import env_rank_world as dist_env_rank_world  # noqa: E402
@@ -31,7 +31,7 @@ from .dist import shard_range as dist_shard_range        # noqa: E402
 
 
 def _load_dataset(dataset):
-    """Returns (tables for TrainData, validation CSR pair, n_items, generator tuple)."""
+    """Returns (tables for TrainData, validation CSR pair, n_items, generator tuple, niche item ids)."""
     if dataset.endswith(".npz"):
         g = np.load(dataset)
         n_items = int(g["n_items"])
@@ -39,7 +39,7 @@ def _load_dataset(dataset):
         vad = (g["vad_tr_indptr"], g["vad_tr_indices"].astype(np.int32), g["vad_te_indptr"], g["vad_te_indices"].astype(np.int32))
         vae = MultiVAE([200, 600, n_items], lam=0.0, random_seed=98765)
         out, loss, params = vae.build_graph()
-        return tabs, vad, n_items, (vae, out, loss, params, [200, 600, n_items], 20000, 0.2)
+        return tabs, vad, n_items, (vae, out, loss, params, [200, 600, n_items], 20000, 0.2), np.sort(g["niche_tags"].astype(np.int64))
     DATA_DIR = dataset + "/"
     show2id_path = DATA_DIR + "item2id.txt"
     niche_tags_path = DATA_DIR + "niche_items.txt"
@@ -77,7 +77,7 @@ def _load_dataset(dataset):
                                  USER_TAGS_TO_SAMPLE, ITEM_FEATURE_DICT, n_items)
     vad_data_tr.sort_indices(); vad_data_te.sort_indices()
     vad = (vad_data_tr.indptr, vad_data_tr.indices, vad_data_te.indptr, vad_data_te.indices)
-    return tabs, vad, n_items, generator(pro_dir)
+    return tabs, vad, n_items, generator(pro_dir), np.asarray(sorted(NICHE_TAGS), dtype=np.int64)
 
 
 def _dist_setup():
@@ -110,7 +110,8 @@ def train_GAN(h0_size, h1_size, h2_size, h3_size, NUM_EPOCH, NUM_SUB_EPOCHS, BAT
     if save and not os.path.exists(output_path):
         os.makedirs(output_path)
 
-    tabs, vad, n_items, gen = _load_dataset(dataset)
+    tabs, vad, n_items, gen, niche_tags = _load_dataset(dataset)
+    item_pop = np.bincount(np.asarray(tabs["indices"], dtype=np.int64), minlength=n_items)   # training interactions per item
     generator_network, generator_out, g_vae_loss, g_params, p_dims, total_anneal_steps, anneal_cap = gen
     if world > 1:
         if BATCH_SIZE % world != 0:
@@ -195,13 +196,14 @@ def train_GAN(h0_size, h1_size, h2_size, h3_size, NUM_EPOCH, NUM_SUB_EPOCHS, BAT
                 log("global-epoch:%s, generator-epoch:%s, g_loss:%.5f (vae_loss: %.5f + gan_loss: %.5f, anneal: %.5f)"
                     % (i, j_gen, L["g_loss"], L["vae_loss"], L["gan_loss"], L["anneal"]))
         log("")
-        m = engine.evaluate(vad[0], vad[1], vad[2], vad[3], k=100, recall_ks=(20, 50))   # train.py:333-348
+        m = engine.evaluate(vad[0], vad[1], vad[2], vad[3], k=100, recall_ks=(20, 50), niche=niche_tags, item_pop=item_pop)   # train.py:333-348
         ndcg_vad, recall_at_20, recall_at_50 = m["ndcg@100"], m["recall@20"], m["recall@50"]
         log("global-epoch:", i, "gen-epoch:", j_gen, "Vad: NDCG:", np.mean(ndcg_vad), "Recall@20:", np.mean(recall_at_20), "Recall@50:",
             np.mean(recall_at_50), "Num_users:", len(ndcg_vad), len(recall_at_20), len(recall_at_50))
         log("")
         rec = dict(epoch=i, ndcg=float(np.mean(ndcg_vad)), r20=float(np.mean(recall_at_20)), r50=float(np.mean(recall_at_50)),
                    d_loss=curr_d_loss)
+        rec.update(longtail_summary(m))
         if diag:
             rec.update(sp_mean=float(np.mean(dg["sp"])) if dg["sp"] else None, ybar_mean=float(np.mean(dg["ybar"])) if dg["ybar"] else None,
                        vae_loss_mean=float(np.mean(dg["vae"])) if dg["vae"] else None, gan_loss_mean=float(np.mean(dg["gan"])) if dg["gan"] else None)
